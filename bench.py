@@ -6,25 +6,27 @@ Workload (BASELINE.json configs[1]): citylearn_challenge_2022_phase_all, 17 buil
 A "step" is one environment time step of all 17 x 4096 units of a rank: actions in, state update, district sums, reward,
 observation at t+1 out.  Metric: building-env steps / s (whole job, all ranks).
 
-  value     device-resident: R back-to-back `cl_rollout` launches of EXACTLY K steps each (actions [K,E,A] already in HBM, every
-            step writes its own observation / reward slab, so a launch's K * 7.8 MB output stream is larger than the 126 MB L2),
-            each launch bracketed by CUDA events on the launch stream; the launches are queued without host synchronisation, so
-            host launch latency is outside the brackets of all but the first.  `value` / `ms_per_step` come from the MEDIAN
-            launch (max over ranks); min / max / first are reported beside it.
+  value     device-resident: the timed region is exactly K = --steps steps, ONE `cl_rollout` launch after W = --warmup untimed
+            steps (actions [K,E,A] already in HBM, every step writes its own observation / reward slab, so the launch's K * 7.8 MB
+            output stream is larger than the 126 MB L2 for K >= 17), bracketed by CUDA events on the launch stream (max over
+            ranks); both launches are queued behind ~10 ms of device writes, so the timed one runs under sustained memory load
+            and host launch latency stays outside the bracket (see `timed_rollout`).
+            `--dump-outputs DIR` writes what that launch computed for its last step (see `dump_outputs`).
   e2e       the public API with HOST buffers, K steps: env.step_host(ndarray) -> ONE native call per step (cl_step_host): this step's
             [E, A] actions wait in page-locked host memory and are read over PCIe by the step kernel, the rewards + the observation
             row (reference-parity observation rows are identical for every env, so one row crosses PCIe and the host gets a
             broadcast view) are written back to page-locked host memory by the kernels, then the stream is synchronised.
             `e2e_dma_copies` is the same loop with cudaMemcpyAsync H2D / D2H around the kernel, `e2e_full_observations` the loop with
-            the full [E, L] observation copy, `e2e_rollout_host` K steps per call.
+            the full [E, L] observation copy, `e2e_rollout_host` one call of K steps.
   roofline  HBM: bytes a rollout launch MOVES (actions + observations + rewards + district sums; the unit state stays in
-            registers between the steps of a launch) / median launch duration.
+            registers between the steps of a launch) / launch duration.
   cpu_baseline  the UNMODIFIED reference (oracle/_ref, installed by oracle/build_ref.py) on one host core, when present; else the
             NumPy oracle port.
   extra     (N = 1, or --extras; C4 and C5 at every N) BASELINE configs[4] (C5: closed loop with an on-device policy, 32 768 envs in total),
             BASELINE configs[2] (C3: 3 LSTM buildings x 65 536 envs, MARL; LSTM cell on the tensor cores), configs[3] per-GPU share (C4: synthetic 1024 buildings x 1024 envs, full-year rollout) and configs[1] with
             stale_observations=False (fresh observations) ride on the same JSON line under "extra"; at N > 1 also the building-sharded
             district (district sums completed inside the step kernel over NVLink peer memory vs the NCCL two-phase variant).
+            The extras keep their own fixed step counts; --steps sets those of configs[1] (value, e2e, fresh observations).
 
 `--impl reference` times the reference's own CPU step on all host cores (one process per core, one env each; oracle/_ref when it
 travelled with the snapshot, else the oracle port) and prints the same line with "impl": "reference".
@@ -287,6 +289,43 @@ def timed_rollouts(env, torch, acts, obs, rew, dst, K: int, R: int, reset_every:
     return [a.elapsed_time(b) for a, b in ev]
 
 
+def timed_rollout(env, torch, acts, obs, rew, dst, K: int, W: int):
+    """From a reset: W untimed warm-up steps in one launch, then ONE `cl_rollout` launch of exactly K steps bracketed by CUDA events on
+    the launch stream.  Returns (milliseconds, kernel launches inside the bracket).
+
+    Both launches are queued behind ~10 ms of writes to the output buffers and nothing synchronises the host in between, so the
+    timed launch starts while the device is under sustained memory load, right after the warm-up launch, and the host's launch
+    latency stays outside the bracket.  Measured on B200 (1000 W): after 1 ms of idle HBM the same launch runs 1.5 % slower
+    (17 x 4096 envs, K = 100) than under sustained load, the state a training loop stepping the env sees."""
+    env.reset()
+    nbytes = sum(t.numel() * t.element_size() for t in (obs, rew, dst))
+    for _ in range(min(2000, 1 + int(10e-3 * 6e12 / nbytes))):
+        obs.zero_(); rew.zero_(); dst.zero_()
+    env.rollout(acts[:W].contiguous(), obs[:W], rew[:W], dst[:W])
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    n0 = env.gpu_launches
+    e0.record()
+    env.rollout(acts[:K].contiguous(), obs[:K], rew[:K], dst[:K])
+    e1.record()
+    torch.cuda.synchronize(env.device)
+    return e0.elapsed_time(e1), env.gpu_launches - n0
+
+
+def dump_outputs(out_dir, arrays, budget=64 << 20, seed=0):
+    """Write each [E, ...] array as `out_dir/<name>.npy`.  Above `budget` bytes in all, every array keeps the same rows: a fixed sample
+    of the envs drawn with `seed`, in ascending order."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    n_envs = len(next(iter(arrays.values())))
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    if n_envs * row_bytes > budget:
+        keep = np.sort(np.random.default_rng(seed).choice(n_envs, budget // row_bytes, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    for name, a in arrays.items():
+        np.save(out / f'{name}.npy', a)
+
+
 def median(xs):
     ys = sorted(xs)
     return ys[len(ys) // 2]
@@ -297,21 +336,19 @@ def timing_summary(ms, K):
             'max_us_per_step': 1e3 * max(ms) / K, 'first_launch_us_per_step': 1e3 * ms[0] / K}
 
 
-def extra_fresh_c2(torch, dev, precision, K, R, peak):
+def extra_fresh_c2(torch, dev, precision, K, W, peak):
     """BASELINE configs[1] with stale_observations=False: observations carry soc / net of the step (per-env row images)."""
     from citylearn_b200 import CityLearnEnv
     E = ENVS_PER_GPU
     env = CityLearnEnv(DATASET, num_envs=E, device=dev, precision=precision, stale_observations=False)
     B, A, L = env.spec.n_buildings, env.spec.action_dim, env._obs_dim
-    acts = torch.rand((K, E, A), device=dev) * 2 - 1
-    obs = torch.empty((K, E, L), device=dev); rew = torch.empty((K, E, B), device=dev); dst = torch.empty((K, E, 3), device=dev)
-    env.reset()
-    timed_rollouts(env, torch, acts, obs, rew, dst, K, 2)
-    ms = timed_rollouts(env, torch, acts, obs, rew, dst, K, R)
-    m = median(ms)
+    N = max(K, W)
+    acts = torch.rand((N, E, A), device=dev) * 2 - 1
+    obs = torch.empty((N, E, L), device=dev); rew = torch.empty((N, E, B), device=dev); dst = torch.empty((N, E, 3), device=dev)
+    m, _ = timed_rollout(env, torch, acts, obs, rew, dst, K, W)
     bpu = bytes_per_unit(precision, L / B, A / B, B)
     out = {'workload': f'{DATASET}: {B} x {E} envs, stale_observations=False (fresh observations)', 'ms_per_step': m / K,
-           'value': B * E * K / (m * 1e-3), 'unit': UNIT, 'timing': timing_summary(ms, K), 'table_path': bool(env._h.geometry()),
+           'value': B * E * K / (m * 1e-3), 'unit': UNIT, 'table_path': bool(env._h.geometry()),
            'roofline': {'bound': 'hbm', 'achieved': bpu * B * E * K / (m * 1e-3) / 1e9, 'peak': peak, 'unit': 'GB/s',
                         'frac': bpu * B * E * K / (m * 1e-3) / 1e9 / peak, 'bytes_per_unit': bpu}}
     env.close()
@@ -518,9 +555,10 @@ def main():
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--precision', default='fp64', choices=['fp64', 'fp32'])
     ap.add_argument('--envs', type=int, default=ENVS_PER_GPU, help='parallel envs per GPU')
-    ap.add_argument('--repeats', type=int, default=50, help='back-to-back K-step launches in the timed region (median reported)')
     ap.add_argument('--extras', default='auto', choices=['auto', 'all', 'none'], help="C3 / C4 / fresh-observation numbers under 'extra' (auto: N = 1 all, N > 1 C4 only)")
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write the observations [E, L], rewards [E, B] and district '
+                    'sums [E, 3] of the last timed step (rank 0, float32) as DIR/<name>.npy; above 64 MB in all, a fixed seeded sample of the envs')
     args = ap.parse_args()
     if args.impl == 'reference':
         return run_reference(args)
@@ -543,7 +581,6 @@ def main():
     B, A, L = env.spec.n_buildings, env.spec.action_dim, env._obs_dim
     T1 = env.time_steps - 1
     assert W + K <= T1, 'steps + warmup must fit in one episode'
-    R = max(3, min(args.repeats, (T1 - W) // K))
 
     # ---------------- device-resident throughput ----------------
     g = torch.Generator(device=dev).manual_seed(1234 + rank)
@@ -551,9 +588,6 @@ def main():
     obs = torch.empty((max(K, W), E, L), device=dev)
     rew = torch.empty((max(K, W), E, B), device=dev)
     dst = torch.empty((max(K, W), E, 3), device=dev)
-    env.reset()
-    env.rollout(acts[:W].contiguous(), obs[:W], rew[:W], dst[:W])                 # W warm-up steps (untimed)
-    torch.cuda.synchronize(dev)
     peaks = {}
     try:
         peaks = json.loads((ROOT / 'MEASURED_PEAKS.json').read_text())
@@ -565,13 +599,12 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    launches0 = env.gpu_launches
     torch.cuda.synchronize(dev)
-    a_k, o_k, r_k, d_k = acts[:K].contiguous(), obs[:K], rew[:K], dst[:K]
-    launch_ms = timed_rollouts(env, torch, a_k, o_k, r_k, d_k, K, R)                # R launches of EXACTLY K steps each
-    launches = env.gpu_launches - launches0
-    ms_med = median(launch_ms)
-    t = torch.tensor([ms_med], device=dev, dtype=torch.float64)
+    ms_launch, launches = timed_rollout(env, torch, acts, obs, rew, dst, K, W)    # W untimed warm-up steps, then ONE launch of K steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'observations': obs[K - 1].cpu().numpy(), 'rewards': rew[K - 1].cpu().numpy(),
+                                         'district': dst[K - 1].cpu().numpy()})
+    t = torch.tensor([ms_launch], device=dev, dtype=torch.float64)
     if world > 1:
         dist.barrier()
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -618,12 +651,10 @@ def main():
     blk = np.random.RandomState(9 + rank).uniform(-1, 1, size=(K, E, A)).astype('float32')
     env.rollout_host(blk)
     torch.cuda.synchronize(dev)
-    tb = []
-    for _ in range(3):
-        if env.time_step + K > T1:
-            env.reset()
-        t0 = time.perf_counter(); env.rollout_host(blk); tb.append(time.perf_counter() - t0)
-    blk_s = torch.tensor([median(tb)], device=dev, dtype=torch.float64)
+    if env.time_step + K > T1:
+        env.reset()
+    t0 = time.perf_counter(); env.rollout_host(blk)
+    blk_s = torch.tensor([time.perf_counter() - t0], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(blk_s, op=dist.ReduceOp.MAX)
     e2e_value = world * units_per_step * K / (e2e_ms * 1e-3)
@@ -649,7 +680,7 @@ def main():
         if rank == 0:
             with torch.cuda.device(dev):
                 fma_peak = _native.measure_fma_peak()
-            guarded('fresh_observations_c2', lambda: extra_fresh_c2(torch, dev, args.precision, K, min(R, 20), peak))
+            guarded('fresh_observations_c2', lambda: extra_fresh_c2(torch, dev, args.precision, K, W, peak))
             guarded('c3_lstm_marl', lambda: extra_c3(torch, dev, args.precision, fma_peak))
     if want != 'none':
         guarded('c4_wide_year', lambda: extra_c4(torch, dev, args.precision, peak, world, dist))
@@ -662,10 +693,10 @@ def main():
 
     bpu = bytes_per_unit(args.precision, L / B, A / B, B, rollout=True)
     bpu_step = bytes_per_unit(args.precision, L / B, A / B, B, rollout=False)
-    # the timed region is R launches of the rollout kernel, K steps each: algorithmic bytes per launch = K steps x bytes a step moves;
-    # duration = the median launch (CUDA events on the launch stream)
+    # the timed region is one launch of the rollout kernel, K steps: algorithmic bytes per launch = K steps x bytes a step moves;
+    # duration = CUDA events on the launch stream
     bytes_per_launch = bpu * units_per_step * K
-    achieved = bytes_per_launch / (ms_med * 1e-3) / 1e9
+    achieved = bytes_per_launch / (ms_launch * 1e-3) / 1e9
     traffic = None
     traffic_note = None
     try:
@@ -697,14 +728,13 @@ def main():
                    'precision': args.precision + (' (float64 intermediates, float32 storage: the reference\'s own flow, bit-exact)' if args.precision == 'fp64'
                                                   else ' (plain float arithmetic: within 1e-4 scaled-relative of the reference, not the 1e-5 target)'),
                    'mode': f'cl_rollout: ONE persistent kernel launch advances all K = {K} steps (state in registers, TMA row ring), actions pre-resident in HBM',
-                   'timed_region': f'{R} back-to-back launches of exactly K steps, one CUDA-event pair each on the launch stream; value = median launch, max over ranks',
+                   'timed_region': 'one launch of exactly K steps after the warm-up, one CUDA-event pair on the launch stream; max over ranks',
                    'l2': f'every step writes its own obs/reward slab: {K} x {bpu * units_per_step / 1e6:.1f} MB per launch vs 126 MB L2',
                    'envs_sharded_across_gpus': True, 'collectives_on_step_path': 0},
-        'timing': timing_summary(launch_ms, K),
         'roofline': {'bound': 'hbm', 'achieved': achieved, 'peak': peak, 'unit': 'GB/s', 'frac': achieved / peak, 'traffic': traffic, 'traffic_source': traffic_note,
                      'kernel': 'advance_kernel', 'bytes_per_unit': bpu, 'bytes_per_unit_single_step_launch': bpu_step,
                      'bytes_per_step': bpu * units_per_step, 'bytes_per_launch': bytes_per_launch, 'steps_per_launch': K,
-                     'avg_launch_us': ms_med * 1e3, 'peak_source': 'MEASURED_PEAKS.json hbm_gbs' if peaks else 'fallback 6650'},
+                     'avg_launch_us': ms_launch * 1e3, 'peak_source': 'MEASURED_PEAKS.json hbm_gbs' if peaks else 'fallback 6650'},
         'cpu_baseline': cpu,
         'e2e': {'value': e2e_value, 'unit': UNIT, 'h2d_bytes_per_step': E * A * 4, 'd2h_bytes_per_step': L * 4 + E * B * 4,
                 'ms_per_step': e2e_ms / K, 'api': 'CityLearnEnv.step_host(ndarray) -> cl_step_host, one native call per step: the step kernel reads the [E, A] actions from page-locked host memory and writes the rewards + the observation row all envs share back to it over PCIe (in place), stream sync'},

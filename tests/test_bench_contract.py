@@ -47,3 +47,40 @@ def test_b200_arm_has_no_cpu_fallback():
     r = run('--steps', '1', '--warmup', '1', '--no-cpu-baseline')
     assert r.returncode != 0
     assert 'CUDA' in (r.stderr + r.stdout)
+
+
+def test_dump_outputs_samples_the_same_envs_of_every_array(tmp_path):
+    import numpy as np
+    from bench import dump_outputs
+    E = 1000
+    arrays = {'a': np.arange(E * 6, dtype='float32').reshape(E, 6), 'b': np.arange(E, dtype='float64')}
+    dump_outputs(tmp_path / 'full', arrays)
+    for k, v in arrays.items():
+        assert np.array_equal(np.load(tmp_path / 'full' / f'{k}.npy'), v)
+    dump_outputs(tmp_path / 'cut', arrays, budget=100 * 32)            # 32 bytes per env: 100 envs fit
+    a, b = np.load(tmp_path / 'cut' / 'a.npy'), np.load(tmp_path / 'cut' / 'b.npy')
+    assert a.shape == (100, 6) and a.dtype == np.float32 and b.dtype == np.float64
+    assert np.array_equal(a[:, 0] / 6, b) and np.all(np.diff(b) > 0)
+    dump_outputs(tmp_path / 'again', arrays, budget=100 * 32)
+    assert np.array_equal(np.load(tmp_path / 'again' / 'b.npy'), b)
+
+
+@pytest.mark.gpu
+def test_b200_arm_times_exactly_the_requested_steps_and_dumps_them(tmp_path):
+    """Two runs with the same arguments dump the same last-step outputs of the one timed K-step launch."""
+    import numpy as np
+    E, K = 64, 7
+    flags = ['--steps', str(K), '--warmup', '3', '--envs', str(E), '--extras', 'none', '--no-cpu-baseline']
+    dumps = []
+    for i in range(2):
+        r = run(*flags, '--dump-outputs', str(tmp_path / str(i)))
+        assert r.returncode == 0, r.stderr[-400:]
+        j = json.loads([ln for ln in r.stdout.splitlines() if ln.strip().startswith('{')][0])
+        assert j['steps'] == K and j['gpu_launches'] == 1 and j['roofline']['steps_per_launch'] == K
+        dumps.append({n: np.load(tmp_path / str(i) / f'{n}.npy') for n in ('observations', 'rewards', 'district')})
+    obs, rew, dst = dumps[0]['observations'], dumps[0]['rewards'], dumps[0]['district']
+    assert obs.dtype == rew.dtype == dst.dtype == np.float32
+    assert obs.shape == (E, 476) and rew.shape == (E, 17) and dst.shape == (E, 3)
+    assert np.isfinite(rew).all() and np.isfinite(dst).all()
+    for n in dumps[0]:
+        assert np.array_equal(dumps[0][n], dumps[1][n], equal_nan=True), n
